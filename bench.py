@@ -6,6 +6,7 @@ A "step" is one full ``log_probability``: kernel-matrix build fused into the blo
 forward triangular solve, log-determinant and |alpha|^2 reductions.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload dense|quasisep]
+                  [--dump-outputs DIR]
 
 * ``value``  : device-timed throughput with X / diag / y already resident in HBM.
 * ``e2e``    : the same metric through the public API ``GaussianProcess(kernel, X, diag=...).log_probability(y)``
@@ -38,6 +39,7 @@ if ROOT not in sys.path:
 N_DENSE = 65536
 NDIM = 3
 SEED = 49382
+OUTPUTS = {}     # name -> what a timed path returned in its last step (written by --dump-outputs)
 
 
 def make_dense_problem(n, rank=0):
@@ -311,18 +313,20 @@ def run_ours(args, rank, local_rank, world):
     if rank == 0:
         sampler.start()
     ms, logp = timed(step_device, args.steps, per_step_ms)
+    OUTPUTS["log_probability"] = logp
     clocks = sampler.stop() if rank == 0 else None
     prof = ctx.profile(reset=True)
     ctx.set_option("profile", 0)
     launches = ctx.launch_count() - l0
 
     # e2e through the public API with host buffers
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     if args.quick:                       # tuning sweeps only: the line is then NOT a valid bench line (no e2e, no baseline)
         ms_e2e, logp_e2e = float("nan"), float("nan")
     else:
         step_e2e()
         ms_e2e, logp_e2e = timed(step_e2e, e2e_steps)
+        OUTPUTS["log_probability_e2e"] = logp_e2e
 
     # ---- the other BASELINE configs, attached to the one line the driver parses --------------------------------------
     sub_records, sharded = {}, None
@@ -331,7 +335,7 @@ def run_ours(args, rank, local_rank, world):
         if world > 1:
             # BASELINE config 3: ONE factorisation sharded over all ranks (collective: every rank takes part)
             try:
-                sharded = measure_sharded(args, ctx, rank, local_rank, world, steps=max(1, min(args.steps, 2)), warmup=1)
+                sharded = measure_sharded(args, ctx, rank, local_rank, world, warmup=1)
             except Exception as e:  # noqa: BLE001
                 sharded = {"error": str(e)[:300]}
         elif rank == 0:
@@ -434,7 +438,7 @@ def _hbm_peak():
         return 6650.0, "fallback 6.65 TB/s (B200_PROFILING.md)"
 
 
-def measure_quasisep(args, ctx, local_rank, n=10_000_000, steps=None, warmup=3, opts=()):
+def measure_quasisep(args, ctx, local_rank, n=10_000_000, warmup=3, opts=()):
     """BASELINE config 4: SHO + Matern-3/2 (J = 4) on a sorted 1-D series of N = 1e7 points, one GPU.
     `value`: device-resident inputs through b200gp_qs_log_probability_dev; `e2e`: GaussianProcess(...).log_probability(y)
     with host buffers.  The C restatement of the sequential recursion (oracle/csrc) checks the FULL series."""
@@ -443,7 +447,7 @@ def measure_quasisep(args, ctx, local_rank, n=10_000_000, steps=None, warmup=3, 
     from tinygp_b200 import GaussianProcess, _cabi
     from tinygp_b200.kernels import quasisep as Q
 
-    steps = steps or max(3, min(args.steps, 10))
+    steps = args.steps
     stream = torch.cuda.current_stream()
     for kv in opts:
         key, _, val = kv.partition("=")
@@ -487,22 +491,19 @@ def measure_quasisep(args, ctx, local_rank, n=10_000_000, steps=None, warmup=3, 
     l0 = ctx.launch_count()
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms_cal, _ = timed(step_device, 10)
-    reps = max(steps, int(2000.0 / max(ms_cal / 10.0, 1e-3)))   # a step is ~1 ms: ~2 s of them so that nvidia-smi samples the clocks
-    ctx.profile(reset=True)
-    l0 = ctx.launch_count()
-    ms, logp = timed(step_device, reps)
+    ms, logp = timed(step_device, steps)
     clocks = sampler.stop()
     prof = ctx.profile(reset=True)
     ctx.set_option("profile", 0)
     launches = ctx.launch_count() - l0
     step_e2e()
-    e2e_steps = 2
+    e2e_steps = steps
     ms_e2e, logp_e2e = timed(step_e2e, e2e_steps)
+    OUTPUTS.update(quasisep_log_probability=logp, quasisep_log_probability_e2e=logp_e2e)
     J = kernel.state_dim()
     alg_bytes = 8.0 * n * (3 + 1 + J)          # read t, diag, y ; write c, w   (SURVEY 8d: 64 B/point at J=4)
     hbm_peak, src = _hbm_peak()
-    achieved = alg_bytes * reps / (prof["qs_ms"] * 1e-3) / 1e9
+    achieved = alg_bytes * steps / (prof["qs_ms"] * 1e-3) / 1e9
     # parity at FULL size: the C restatement of ops.py:352-365,463-472 on all N points (1 core)
     from oracle import cref, tinygp_np as o
     ko = o.qs.SHO(1.5, 3.0, 1.8) + o.qs.Matern32(1.5, 0.9)
@@ -512,8 +513,8 @@ def measure_quasisep(args, ctx, local_rank, n=10_000_000, steps=None, warmup=3, 
     t_cpu = time.perf_counter() - t0
     del d_, p_, q_, a_
     return {
-        "metric": "log_probability/sec", "value": reps / (ms * 1e-3), "unit": "logp/s", "n_gpus": 1,
-        "steps": reps, "warmup": warmup, "ms_per_step": ms / reps, "higher_is_better": True, "dtype": "f64", "data": "synthetic",
+        "metric": "log_probability/sec", "value": steps / (ms * 1e-3), "unit": "logp/s", "n_gpus": 1,
+        "steps": steps, "warmup": warmup, "ms_per_step": ms / steps, "higher_is_better": True, "dtype": "f64", "data": "synthetic",
         "config": {"workload": f"quasisep SHO+Matern32 (J=4) N={n} log_probability", "diag": 0.1, "seed": 49384,
                    "options": list(opts), "l2": "working set 0.64 GB > 126 MB L2"},
         "logp": logp, "logp_e2e": logp_e2e,
@@ -530,7 +531,7 @@ def measure_quasisep(args, ctx, local_rank, n=10_000_000, steps=None, warmup=3, 
         "e2e": {"value": e2e_steps / (ms_e2e * 1e-3), "unit": "logp/s", "h2d_bytes_per_step": int(3 * 8 * n),
                 "d2h_bytes_per_step": 16,
                 "note": "pinned host buffers; 240 MB over PCIe per call (t, diag, y) bound e2e at ~200 logp/s whatever the kernels do"},
-        "gpu_launches": int(launches), "kernel_ms_per_step": {"qs": prof["qs_ms"] / reps},
+        "gpu_launches": int(launches), "kernel_ms_per_step": {"qs": prof["qs_ms"] / steps},
     }
 
 
@@ -541,12 +542,12 @@ def run_quasisep(args, rank, local_rank, world):
     if args.qs_chunk:
         ctx.set_option("qs_chunk", args.qs_chunk)
     n = args.n if args.n != N_DENSE else 10_000_000
-    line = measure_quasisep(args, ctx, local_rank, n=n, steps=args.steps, warmup=args.warmup, opts=args.opt)
+    line = measure_quasisep(args, ctx, local_rank, n=n, warmup=args.warmup, opts=args.opt)
     line.update({"scaling": "weak", "vs_baseline": None})
     print(json.dumps(line), flush=True)
 
 
-def measure_batched(args, ctx, local_rank, rank=0, world=1, n=4096, steps=2, warmup=1):
+def measure_batched(args, ctx, local_rank, rank=0, world=1, n=4096, warmup=1):
     """BASELINE config 5: 1024 independent N=4096 ExpSquared problems (32 x 32 hyper-parameter grid), sharded
     128 per GPU at 8 GPUs -- replicas only, no data-path collective."""
     import torch
@@ -554,6 +555,7 @@ def measure_batched(args, ctx, local_rank, rank=0, world=1, n=4096, steps=2, war
     from tinygp_b200 import _cabi, kernels
 
     stream = torch.cuda.current_stream()
+    steps = args.steps
     nprob = 1024
     rng = np.random.default_rng(49385)
     X = np.ascontiguousarray(rng.uniform(0, 8, (n, 3)))
@@ -589,6 +591,7 @@ def measure_batched(args, ctx, local_rank, rank=0, world=1, n=4096, steps=2, war
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     t = float(ms.item()) * 1e-3
+    OUTPUTS["batched_log_probability"] = out.copy()
     # parity on the corners of the grid this rank holds (oracle: LAPACK at N = 4096, ~1 s each)
     from oracle import tinygp_np as o
     checks = []
@@ -624,7 +627,7 @@ def run_batched(args, rank, local_rank, world):
     for kv in args.opt:                            # tuning experiments: --opt nb_batched=1024 ...
         key, _, val = kv.partition("=")
         ctx.set_option(key, int(val))
-    line = measure_batched(args, ctx, local_rank, rank, world, n=n, steps=args.steps, warmup=args.warmup)
+    line = measure_batched(args, ctx, local_rank, rank, world, n=n, warmup=args.warmup)
     if args.opt:
         line["config"]["options"] = list(args.opt)
     if rank == 0:
@@ -633,7 +636,7 @@ def run_batched(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
-def measure_sharded(args, ctx, rank, local_rank, world, n=131072, steps=2, warmup=1, slices=None):
+def measure_sharded(args, ctx, rank, local_rank, world, n=131072, warmup=1, slices=None):
     """BASELINE config 3: ONE dense log_probability sharded over the GPUs.  Kernel 1.5*Matern52(2.0) +
     0.7*RationalQuadratic(1.5, alpha=1.5), both with the Euclidean metric (the L1 defaults are indefinite in 3-D, see
     DESIGN.md section 2), N = 131072 by default.  Strong scaling.  Collective: every rank must call this."""
@@ -642,6 +645,7 @@ def measure_sharded(args, ctx, rank, local_rank, world, n=131072, steps=2, warmu
     from tinygp_b200 import kernels, multigpu
 
     ctx.set_option("nb", args.nb)
+    steps = args.steps
     rng = np.random.default_rng(49383)
     side = 25.0 * (n / 131072.0) ** (1.0 / 3.0)
     X = np.ascontiguousarray(rng.uniform(0.0, side, (n, NDIM)))
@@ -681,6 +685,7 @@ def measure_sharded(args, ctx, rank, local_rank, world, n=131072, steps=2, warmu
     ctx.set_option("profile", 0)
     ms = max_over_ranks(e0.elapsed_time(e1), device="cuda")
     t = ms * 1e-3
+    OUTPUTS["sharded_log_probability"] = lp
     line = {
         "metric": "log_probability/sec", "value": steps / t, "unit": "logp/s", "n_gpus": world, "steps": steps,
         "warmup": warmup, "ms_per_step": ms / steps, "higher_is_better": True, "scaling": "strong",
@@ -716,7 +721,7 @@ def run_sharded(args, rank, local_rank, world):
         key, _, val = kv.partition("=")
         ctx.set_option(key, int(val))
     n = 131072 if args.n == N_DENSE else args.n
-    line = measure_sharded(args, ctx, rank, local_rank, world, n=n, steps=args.steps, warmup=args.warmup)
+    line = measure_sharded(args, ctx, rank, local_rank, world, n=n, warmup=args.warmup)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -733,10 +738,19 @@ def _read_traffic(name="syrk_traffic.json", key="dram_bytes_per_launch"):
         return None
 
 
+def dump_outputs(directory):
+    """OUTPUTS as DIR/<name>.npy in float64: with the same arguments the inputs are the same seeded arrays, so two builds
+    can be compared output for output"""
+    os.makedirs(directory, exist_ok=True)
+    for name, value in OUTPUTS.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.asarray(value, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps of every timed leg: the device path, e2e, and the attached configs")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--size", "--n", dest="n", type=int, default=N_DENSE, help="problem size N (use --size under torchrun)")
@@ -753,7 +767,14 @@ def main():
                     help="dense workload: skip the attached sub-records (C4 quasisep, C5 batched; sharded C3 when WORLD_SIZE > 1)")
     ap.add_argument("--opt", action="append", default=[], metavar="KEY=INT",
                     help="library option for tuning runs (b200gp_set_option); dense and quasisep workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what each timed path returned in its last step as "
+                         "DIR/<name>.npy (float64); rank 0's values (its shard of the batched grid); impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a smaller sample of the workload, not the same outputs")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -768,6 +789,8 @@ def main():
             run_quasisep(args, rank, local_rank, world)
     else:
         run_ours(args, rank, local_rank, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs)
 
 
 if __name__ == "__main__":

@@ -26,8 +26,10 @@ class HostBackend:
             pytest.skip("g++ not available")
         if not os.path.exists(OUT) or any(os.path.getmtime(d) > os.path.getmtime(OUT) for d in DEPS):
             os.makedirs(os.path.dirname(OUT), exist_ok=True)
-            subprocess.run([gxx, "-O2", "-std=c++17", "-DQSM_HOSTCHECK", "-fPIC", "-shared", "-x", "c++", SRC, "-o", OUT],
+            tmp = f"{OUT}.{os.getpid()}"     # parallel workers each build their own copy and swap it in whole
+            subprocess.run([gxx, "-O2", "-std=c++17", "-DQSM_HOSTCHECK", "-fPIC", "-shared", "-x", "c++", SRC, "-o", tmp],
                            check=True)
+            os.replace(tmp, OUT)
         lib = ctypes.CDLL(OUT)
         for name, (res, args) in _cabi.SIGNATURES.items():
             if hasattr(lib, name):

@@ -1,10 +1,12 @@
-"""The plugin boundary, literally: the UNMODIFIED reference `tinygp.GaussianProcess` (from /root/reference, over the
-NumPy stand-ins for jax/equinox in tests/golden/jaxshim) driven with `solver=tinygp_b200.adapter.DirectSolver /
-QuasisepSolver`.  tinygp's own gp.py makes every call (constructor with `covariance=`, the six Solver methods, the
-Conditioned kernel calling back into `solve_triangular`); the B200 host layer answers, here over the mock C-ABI
-(tests/hostmock.py) because this container has no GPU and the GPU box has no reference checkout.  Results must equal
-what the reference computes with its own solvers."""
+"""The plugin boundary: `tinygp_b200.adapter.DirectSolver / QuasisepSolver` take tinygp's own kernel and noise objects
+and must give what the reference computes with its own solvers.  tests/golden/adapter_vectors.npz holds, for every
+case, the reference's results and its kernel / noise objects recorded as data (class name, module, field values;
+made by tests/golden/make_golden_adapter.py, which also checks the reference's gp.py driving these solvers).  Here the
+recorded objects are rebuilt as plain attribute holders of the same class and module names, so the adapter translates
+exactly what it is given by tinygp, and a GaussianProcess drives the adapter's solvers.  The host layer runs over the
+mock C-ABI (tests/hostmock.py), so no GPU is needed."""
 
+import json
 import os
 import sys
 from ctypes import c_void_p
@@ -16,132 +18,124 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.join(HERE, "golden"))
 
-import refimport  # noqa: E402
-
-if not refimport.available():
-    pytest.skip("the reference checkout (/root/reference) is not present on this machine", allow_module_level=True)
-
+import adaptercases as C  # noqa: E402
 import hostmock  # noqa: E402
-from tinygp_b200 import _cabi, adapter  # noqa: E402
+from tinygp_b200 import GaussianProcess, _cabi, adapter, noise  # noqa: E402
+
+GOLD = np.load(os.path.join(HERE, "golden", "adapter_vectors.npz"))
+TREES = json.loads(str(GOLD["trees"]))
+DENSE, QS = C.DENSE, C.QS
+
+
+def foreign(node):
+    """a recorded reference object: same class name, module and field values, no behaviour of its own"""
+    if isinstance(node, list):
+        return [foreign(v) for v in node]
+    if not isinstance(node, dict):
+        return node
+    if "array" in node:
+        return GOLD[node["array"]]
+    obj = type(node["class"], (), {"__module__": node["module"]})()
+    for name, value in node["fields"].items():
+        setattr(obj, name, foreign(value))
+    return obj
+
+
+def objects(case):
+    return {name: foreign(tree) for name, tree in TREES[case].items()}
 
 
 @pytest.fixture()
-def tinygp(monkeypatch):
-    saved = list(sys.path)
-    mods = set(sys.modules)
-    tg = refimport.install()
+def mock_device():
     lib = hostmock.MockLib()
     ctx = _cabi.Context.__new__(_cabi.Context)
     ctx.lib, ctx.handle, ctx.device = lib, c_void_p(1), -1
     previous = _cabi._ctx
     _cabi.set_context(ctx)
     try:
-        yield tg
+        yield
     finally:
         _cabi.set_context(previous)
-        sys.path[:] = saved
-        for m in set(sys.modules) - mods:          # do not leak the stand-in `jax` into other test modules
-            if m.split(".")[0] in ("jax", "equinox", "tinygp"):
-                del sys.modules[m]
 
 
-def _close(a, b, tol=1e-9):
-    a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
+def _close(a, key, tol=1e-9):
+    a, b = np.asarray(a, dtype=np.float64), GOLD[key]
     assert a.shape == b.shape and np.all(np.isfinite(b)), "the reference itself must be finite for this comparison"
-    assert np.max(np.abs(a - b)) <= tol * max(1.0, np.max(np.abs(b))), (np.max(np.abs(a - b)))
-
-
-DENSE = [
-    "1.7 * kernels.ExpSquared(0.9)",
-    "kernels.Matern32(1.3, distance=kernels.L2Distance()) + 0.3 * kernels.RationalQuadratic(scale=1.5, alpha=0.8)",
-    "kernels.Exp(1.3) * kernels.ExpSquared(3.0) + 0.05",
-    "transforms.Subspace(0, kernels.ExpSquared(1.2)) + 0.5 * transforms.Linear(np.array([0.7, 1.4]), kernels.Matern52(0.9))",
-]
+    assert np.max(np.abs(a - b)) <= tol * max(1.0, np.max(np.abs(b))), (key, np.max(np.abs(a - b)))
 
 
 @pytest.mark.parametrize("expr", DENSE)
-def test_reference_gaussian_process_with_b200_direct_solver(tinygp, expr):
-    from tinygp import GaussianProcess, kernels, transforms
-    rng = np.random.default_rng(3)
-    X, Xt = rng.uniform(0, 4, (40, 2)), rng.uniform(0, 4, (6, 2))
-    y = np.sin(X[:, 0]) + 0.1 * rng.normal(size=40)
-    k = eval(expr, {"kernels": kernels, "transforms": transforms, "np": np})
-    ref = GaussianProcess(k, X, diag=0.07, mean=0.2)
-    ours = GaussianProcess(k, X, diag=0.07, mean=0.2, solver=adapter.DirectSolver)
+def test_reference_gaussian_process_with_b200_direct_solver(mock_device, expr):
+    p = f"dense{DENSE.index(expr)}/"
+    X, Xt, y = C.dense_inputs()
+    ref = objects(p[:-1])
+    ours = GaussianProcess(adapter.translate_kernel(ref["kernel"]), X, diag=0.07, mean=0.2, solver=adapter.DirectSolver)
     assert isinstance(ours.solver, adapter.DirectSolver)
-    _close(ours.log_probability(y), ref.log_probability(y))
-    _close(ours.variance, ref.variance)
-    _close(ours.covariance, ref.covariance)
+    _close(ours.log_probability(y), p + "log_probability")
+    _close(ours.variance, p + "variance")
+    _close(ours.covariance, p + "covariance")
     lp_o, cond_o = ours.condition(y, Xt, diag=1e-3)
-    lp_r, cond_r = ref.condition(y, Xt, diag=1e-3)
-    _close(lp_o, lp_r)
-    _close(cond_o.loc, cond_r.loc)
-    _close(cond_o.variance, cond_r.variance)          # tinygp's Conditioned kernel calls back into our solve_triangular
-    _close(cond_o.covariance, cond_r.covariance)
-    _close(cond_o.log_probability(np.cos(Xt[:, 0])), cond_r.log_probability(np.cos(Xt[:, 0])))
+    _close(lp_o, p + "cond_log_probability")
+    _close(cond_o.loc, p + "cond_loc")
+    _close(cond_o.variance, p + "cond_variance")        # the Conditioned kernel calls back into our solve_triangular
+    _close(cond_o.covariance, p + "cond_covariance")
+    _close(cond_o.log_probability(np.cos(Xt[:, 0])), p + "cond_log_probability_test")
     mu_o, var_o = ours.predict(y, return_var=True)
-    mu_r, var_r = ref.predict(y, return_var=True)
-    _close(mu_o, mu_r)
-    _close(var_o, var_r)
-    import jax
-    _close(ours.sample(jax.random.PRNGKey(4), shape=(3,)), ref.sample(jax.random.PRNGKey(4), shape=(3,)))
-
-
-QS = [
-    "quasisep.SHO(omega=1.5, quality=3.0, sigma=1.8) + quasisep.Matern32(scale=1.5, sigma=0.9)",
-    "2.0 * quasisep.Matern52(1.2) + quasisep.Celerite(1.1, 0.1, 0.3, 1.5)",
-    "quasisep.Cosine(scale=3.0, sigma=0.7) + quasisep.Exp(scale=2.0, sigma=0.5)",
-]
+    _close(mu_o, p + "predict_mean")
+    _close(var_o, p + "predict_var")
+    _close(ours.sample(C.SAMPLE_SEED, shape=C.SAMPLE_SHAPE), p + "sample")
+    # the solver as tinygp's gp.py constructs and calls it: reference kernel and noise objects in, arrays out
+    solver = adapter.DirectSolver(ref["kernel"], X, ref["noise"])
+    _close(solver.covariance(), p + "covariance")
+    _close(solver.variance(), p + "variance")
+    _close(solver.normalization(), p + "normalization")
+    _close(solver.condition(ref["kernel"], Xt, ref["test_noise"]), p + "solver_condition")
 
 
 @pytest.mark.parametrize("expr", QS)
-def test_reference_gaussian_process_with_b200_quasisep_solver(tinygp, expr):
-    from tinygp import GaussianProcess
-    from tinygp.kernels import quasisep
-    rng = np.random.default_rng(5)
-    t = np.sort(rng.uniform(0, 12, 60))
-    tt = rng.uniform(-1, 13, 5)
-    y = np.sin(t) + 0.1 * rng.normal(size=60)
-    k = eval(expr, {"quasisep": quasisep})
-    ref = GaussianProcess(k, t, diag=0.07)
+def test_reference_gaussian_process_with_b200_quasisep_solver(mock_device, expr):
+    p = f"qs{QS.index(expr)}/"
+    t, tt, y = C.qs_inputs()
+    ref = objects(p[:-1])
+    k = adapter.translate_kernel(ref["kernel"])
     ours = GaussianProcess(k, t, diag=0.07, solver=adapter.QuasisepSolver, parallel=True)
-    _close(ours.log_probability(y), ref.log_probability(y))
-    _close(ours.variance, ref.variance)
+    _close(ours.log_probability(y), p + "log_probability")
+    _close(ours.variance, p + "variance")
     lp_o, cond_o = ours.condition(y, tt, diag=1e-3)
-    lp_r, cond_r = ref.condition(y, tt, diag=1e-3)
-    _close(lp_o, lp_r)
-    _close(cond_o.loc, cond_r.loc)
-    _close(cond_o.variance, cond_r.variance)
-    _close(cond_o.covariance, cond_r.covariance)
+    _close(lp_o, p + "cond_log_probability")
+    _close(cond_o.loc, p + "cond_loc")
+    _close(cond_o.variance, p + "cond_variance")
+    # tinygp's gp.py takes the conditioned variance as kernel(X) + noise.diagonal() (solvers/direct.py:49), the
+    # Conditioned kernel calling back into our solve_triangular
+    _close(cond_o.kernel(tt) + cond_o.noise.diagonal(), p + "cond_variance")
+    _close(cond_o.covariance, p + "cond_covariance")
+    solver = adapter.QuasisepSolver(ref["kernel"], t, ref["noise"], parallel=True)
+    _close(solver.variance(), p + "variance")
+    _close(solver.normalization(), p + "normalization")
+    _close(solver.condition(ref["kernel"], tt, ref["test_noise"]), p + "solver_condition")
     with pytest.raises(ValueError, match="Input coordinates must be sorted"):
         GaussianProcess(k, t[::-1].copy(), diag=0.07, solver=adapter.QuasisepSolver)
 
 
-def test_unsupported_objects_are_refused_loudly(tinygp):
-    from tinygp import GaussianProcess, kernels, noise
+def test_unsupported_objects_are_refused_loudly(mock_device):
     X = np.linspace(0, 1, 5)
     with pytest.raises(NotImplementedError, match="unsupported by the B200"):
-        GaussianProcess(kernels.DotProduct(), X, diag=0.1, solver=adapter.DirectSolver)
+        adapter.DirectSolver(objects("unsupported")["kernel"], X, noise.Diagonal(np.full(5, 0.1)))
 
 
-def test_reference_gaussian_process_with_banded_and_dense_noise(tinygp):
+def test_reference_gaussian_process_with_banded_and_dense_noise(mock_device):
     """the reference's own noise.Banded / noise.Dense objects (noise.py:98-240) through the adapter's solvers"""
-    from tinygp import GaussianProcess, kernels, noise
-    from tinygp.kernels import quasisep
-    rng = np.random.default_rng(8)
-    t = np.sort(rng.uniform(0, 12, 50))
-    tt, y = rng.uniform(-1, 13, 5), np.sin(t)
-    banded = noise.Banded(diag=rng.uniform(0.1, 0.2, 50), off_diags=0.02 * rng.normal(size=(50, 2)))
-    dense = noise.Dense(value=np.asarray(banded + np.zeros((50, 50))))
-    kq = quasisep.Matern32(scale=1.5, sigma=1.8) + quasisep.Exp(scale=0.7)
-    from tinygp.solvers import DirectSolver, QuasisepSolver
-    for k, nz, theirs, solver in ((kq, banded, QuasisepSolver, adapter.QuasisepSolver),
-                                  (kq, banded, DirectSolver, adapter.DirectSolver),
-                                  (kernels.Matern52(1.1), dense, DirectSolver, adapter.DirectSolver)):
-        ref, ours = GaussianProcess(k, t, noise=nz, solver=theirs), GaussianProcess(k, t, noise=nz, solver=solver)
-        _close(ours.log_probability(y), ref.log_probability(y))
-        _close(ours.covariance, ref.covariance)
-        (lp_o, cond_o), (lp_r, cond_r) = ours.condition(y, tt, diag=1e-3), ref.condition(y, tt, diag=1e-3)
-        _close(lp_o, lp_r)
-        _close(cond_o.loc, cond_r.loc)
-        _close(cond_o.covariance, cond_r.covariance)
+    t, tt, y, _, _ = C.banded_inputs()
+    for j, solver in enumerate((adapter.QuasisepSolver, adapter.DirectSolver, adapter.DirectSolver)):
+        p, ref = f"noise{j}/", objects(f"noise{j}")
+        ours = GaussianProcess(adapter.translate_kernel(ref["kernel"]), t, noise=adapter.translate_noise(ref["noise"]),
+                               solver=solver)
+        _close(ours.log_probability(y), p + "log_probability")
+        _close(ours.covariance, p + "covariance")
+        lp_o, cond_o = ours.condition(y, tt, diag=1e-3)
+        _close(lp_o, p + "cond_log_probability")
+        _close(cond_o.loc, p + "cond_loc")
+        _close(cond_o.covariance, p + "cond_covariance")
+        s = solver(ref["kernel"], t, ref["noise"])
+        _close(s.covariance(), p + "covariance")
+        _close(s.normalization(), p + "normalization")

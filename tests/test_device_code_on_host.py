@@ -59,8 +59,10 @@ def lib():
         pytest.skip("nvcc not available")
     if not os.path.exists(OUT) or any(os.path.getmtime(d) > os.path.getmtime(OUT) for d in DEPS):
         os.makedirs(os.path.dirname(OUT), exist_ok=True)
+        tmp = f"{OUT}.{os.getpid()}"     # parallel workers each build their own copy and swap it in whole
         subprocess.run([nvcc, "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-Xcompiler", "-fPIC", "-shared",
-                        "-o", OUT, SRC], check=True)
+                        "-o", tmp, SRC], check=True)
+        os.replace(tmp, OUT)
     return ctypes.CDLL(OUT)
 
 
@@ -135,8 +137,10 @@ def klib():
         pytest.skip("nvcc not available")
     if not os.path.exists(KOUT) or any(os.path.getmtime(d) > os.path.getmtime(KOUT) for d in KDEPS):
         os.makedirs(os.path.dirname(KOUT), exist_ok=True)
+        tmp = f"{KOUT}.{os.getpid()}"
         subprocess.run([nvcc, "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-diag-suppress", "20013",
-                        "-Xcompiler", "-fPIC", "-shared", "-o", KOUT, KSRC], check=True)
+                        "-Xcompiler", "-fPIC", "-shared", "-o", tmp, KSRC], check=True)
+        os.replace(tmp, KOUT)
     return ctypes.CDLL(KOUT)
 
 

@@ -15,8 +15,9 @@ method forwards to the C-ABI-backed solver of ``tinygp_b200.solvers``.
 Scope: eager use.  tinygp decorates ``GaussianProcess._compute_log_prob`` etc. with ``jax.jit`` and traces ``self``,
 so inside real JAX these classes additionally have to be ``equinox.Module``s whose methods go through
 ``jax.pure_callback`` (INTEGRATION.md section 3) -- JAX is not installable in this image, so that last wrapper is
-not built; the contract itself is exercised end to end by tests/test_adapter_with_reference.py, which runs the
-unmodified reference ``GaussianProcess`` with these solvers.
+not built; the Solver interface itself is exercised end to end by tests/golden/make_golden_adapter.py, which runs the
+unmodified reference ``GaussianProcess`` with these solvers, and by tests/test_adapter_with_reference.py against its
+recorded results.
 """
 
 from __future__ import annotations
@@ -124,7 +125,8 @@ class _Adapter:
 
     def condition(self, kernel, X_test, noise):
         Xt = None if X_test is None else np.asarray(X_test, dtype=np.float64)
-        return np.asarray(self.inner.condition(translate_kernel(kernel), Xt, translate_noise(noise)))
+        # asanyarray keeps the ConditionedCovariance tag that tinygp_b200.GaussianProcess reads for the variance
+        return np.asanyarray(self.inner.condition(translate_kernel(kernel), Xt, translate_noise(noise)))
 
 
 class DirectSolver(_Adapter):
